@@ -1,12 +1,12 @@
 #!/usr/bin/env python
 """bench.py — decode tokens/s, Llama-2-7B-shaped Q4_K_M GGUF, batch 1 (BASELINE.json metric, configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one single-token decode pass of the whole hot path: ONE launch of the persistent step kernel (csrc/stream.cuh) whose
 phases are the 129 mat-vecs over 225 weight tensors, 32 attention blocks at a context of 256..511 tokens, the embedding row and the greedy pick.  Workload: synthetic 7B-shaped model (random valid quant blocks in the reference's Q4_K_M tensor mix,
 3.8 GB of weights ≫ the 126 MB L2, so every step streams its inputs from HBM — no L2 flush needed), 256-token prompt
-prefilled untimed, then W warm-up + K timed decode steps.
+prefilled untimed, then W warm-up + K timed decode steps (the context grows past 512 when K needs it).
 
   value     device-timed: K steps replayed as CUDA graphs with the token fed back on the device (the pick phase), CUDA events on the
             launching stream, max over ranks; tokens/s summed over ranks (replicas: one sequence per GPU, weak scaling).  The
@@ -140,6 +140,22 @@ def hbm_peak():
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
 
 
+def context_for(n_tokens):
+    """CTX, or longer when the prompt, warm-up and timed steps do not fit in it (so --steps is never cut short)."""
+    return max(CTX, n_tokens + 1)
+
+
+def dump_outputs(out_dir, llm, tokens):
+    """--dump-outputs: what a caller of the timed path holds after its last step, for comparing two builds output for output
+    (same arguments, same inputs): the greedy tokens of the timed steps, that step's logits and hidden state."""
+    import numpy as np
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / "tokens.npy", np.array(tokens, np.float64))
+    np.save(d / "logits.npy", np.array(llm.logits, np.float32))
+    np.save(d / "embeddings.npy", np.array(llm.embeddings, np.float32))
+
+
 def kv_bytes_per_step(n_layer, n_embd_gqa, t_avg):
     return 2 * n_layer * n_embd_gqa * t_avg * 2 + 2 * n_layer * n_embd_gqa * 2
 
@@ -171,23 +187,28 @@ def run_reference(args, rank, world, barrier):
     from ctransformers_b200 import AutoModelForCausalLM
     cores = os.cpu_count() or 1
     p = ensure_model(0, 1, lambda: None)
-    llm = AutoModelForCausalLM.from_pretrained(str(p), lib=str(REF_SO), context_length=CTX, threads=min(cores, 16))
+    steps = max(1, args.steps)
+    ctx = context_for(PROMPT + 2 * 9 + args.warmup + steps)        # 9: the most thread counts pick_threads tries, 2 evals each
+    llm = AutoModelForCausalLM.from_pretrained(str(p), lib=str(REF_SO), context_length=ctx, threads=min(cores, 16))
     ids = prompt_ids()
     llm.eval(ids, batch_size=256, threads=min(cores, 32))           # untimed prefill, one chunk
     tok = llm.sample(top_k=1, repetition_penalty=1.0, seed=0)
     threads, sweep = pick_threads(llm, tok, cores)
-    steps = max(1, min(args.steps, CTX - PROMPT - args.warmup - 2 * len(sweep) - 1))
     for _ in range(args.warmup):
         llm.eval([tok], threads=threads); tok = llm.sample(top_k=1, repetition_penalty=1.0, seed=0)
     t0 = time.perf_counter()
+    tokens = []
     for _ in range(steps):
         llm.eval([tok], threads=threads); tok = llm.sample(top_k=1, repetition_penalty=1.0, seed=0)
+        tokens.append(tok)
     dt = time.perf_counter() - t0
     v = steps / dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, llm, tokens)
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": v, "unit": "tokens/s", "n_gpus": args.gpus, "steps": steps,
         "warmup": args.warmup, "ms_per_step": 1e3 * dt / steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": DTYPE,
-        "data": "synthetic", "config": workload_config(1),
+        "data": "synthetic", "config": workload_config(1, ctx),
         "cpu_baseline": {"value": v, "unit": "tokens/s", "cores": threads, "kind": "reference", "host_cores": cores, "thread_sweep_s_per_token": sweep,
                          "sample": f"{steps} decode steps at context {PROMPT}+ after a {PROMPT}-token prompt, llm.eval+llm.sample, unmodified reference CPU build (AVX2), {threads} threads (best of the sweep)"},
         "e2e": {"value": v, "unit": "tokens/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -208,7 +229,7 @@ def run_prefill(args, path, rank, world, local, barrier, max_over_ranks, group):
     shape = getattr(synth, WL["shape"])
     ids = np.random.default_rng(1).integers(WL["lo"], shape.n_vocab, n_prompt).tolist()
     ids[0] = 1
-    steps, W = max(1, min(args.steps, 8)), 1
+    steps, W = max(1, args.steps), 1
 
     def once():
         llm._context = []
@@ -249,6 +270,8 @@ def run_prefill(args, path, rank, world, local, barrier, max_over_ranks, group):
         "first_token_after_prompt": int(tok),
     }
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, llm, [tok])
         print(json.dumps(result))
     group.close()
 
@@ -265,10 +288,11 @@ def run_tp(args, path, rank, world, local, barrier, max_over_ranks, group):
         ticket = tensor_parallel_ticket()
     else:
         ticket = None
-    llm = LLM(str(path), config=Config(context_length=CTX), tp=ticket)
-    ids = prompt_ids()
-    steps = max(1, min(args.steps, CTX - PROMPT - args.warmup - 1))
+    steps = max(1, args.steps)
     W = max(args.warmup, 3)
+    ctx = context_for(PROMPT + W + steps)
+    llm = LLM(str(path), config=Config(context_length=ctx), tp=ticket)
+    ids = prompt_ids()
     llm.eval(ids, batch_size=256)
     tok = llm.sample(top_k=1, repetition_penalty=1.0, seed=0)
     for _ in range(W):
@@ -305,8 +329,8 @@ def run_tp(args, path, rank, world, local, barrier, max_over_ranks, group):
     result = {
         "metric": METRIC, "value": steps / (ms / 1e3), "unit": "tokens/s", "n_gpus": world, "steps": steps, "warmup": W, "ms_per_step": ms / steps,
         "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": DTYPE, "data": "synthetic",
-        "config": {"workload": WL["name"] + " (synthetic random quant blocks), batch=1 decode, ctx=512, 256-token prompt then decode", "global_batch": 1,
-                   "ctx": CTX, "prompt": PROMPT, "parallelism": f"tp{world} (column-parallel q/k/v/gate/up, row-parallel wo/down, {2 * shape.n_layer} all-reduces of {shape.n_embd} floats per token over NCCL)",
+        "config": {"workload": WL["name"] + f" (synthetic random quant blocks), batch=1 decode, ctx={ctx}, 256-token prompt then decode", "global_batch": 1,
+                   "ctx": ctx, "prompt": PROMPT, "parallelism": f"tp{world} (column-parallel q/k/v/gate/up, row-parallel wo/down, {2 * shape.n_layer} all-reduces of {shape.n_embd} floats per token over NCCL)",
                    "l2": "each rank streams its GBs of weights per step: inputs exceed the 126 MB L2"},
         "clocks": clocks,
         "e2e": {"value": steps / e2e_s, "unit": "tokens/s", "h2d_bytes_per_step": 16, "d2h_bytes_per_step": 8,
@@ -318,14 +342,16 @@ def run_tp(args, path, rank, world, local, barrier, max_over_ranks, group):
         "greedy_tokens_match_e2e": tokens_dev[:steps] == e2e_tokens[:steps], "ranks_agree": ranks_agree,
     }
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, llm, tokens_dev)
         print(json.dumps(result))
     del llm
     group.close()
 
 
-def workload_config(n):
-    return {"workload": WL["name"] + " (synthetic random quant blocks), batch=1 decode, ctx=512, 256-token prompt then decode",
-            "global_batch": n, "ctx": CTX, "prompt": PROMPT, "parallelism": f"replicas x{n} (one sequence per GPU, no collective)",
+def workload_config(n, ctx):
+    return {"workload": WL["name"] + f" (synthetic random quant blocks), batch=1 decode, ctx={ctx}, 256-token prompt then decode",
+            "global_batch": n, "ctx": ctx, "prompt": PROMPT, "parallelism": f"replicas x{n} (one sequence per GPU, no collective)",
             "l2": "inputs (GBs of weights per step) exceed the 126 MB L2; no flush needed"}
 
 
@@ -339,6 +365,8 @@ def main():
     ap.add_argument("--workload", default="llama2-7b", choices=sorted(WORKLOADS))
     ap.add_argument("--mode", default="replicas", choices=["replicas", "tp"],
                     help="tp: ONE sequence, layer weights tensor-sharded over the ranks (BASELINE configs[4]; implies --workload llama2-13b unless one is given)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (tokens, logits, embeddings)")
     args = ap.parse_args()
     global WL, METRIC, DTYPE
     if args.mode == "tp" and args.workload == "llama2-7b" and "--workload" not in sys.argv:
@@ -372,11 +400,12 @@ def main():
         return run_tp(args, path, rank, world, local, barrier, max_over_ranks, group)
     if args.workload == "prefill2048":
         return run_prefill(args, path, rank, world, local, barrier, max_over_ranks, group)
-    llm = AutoModelForCausalLM.from_pretrained(str(path), context_length=CTX)
+    steps = max(1, args.steps)
+    W = max(args.warmup, 3)
+    ctx = context_for(PROMPT + W + steps)
+    llm = AutoModelForCausalLM.from_pretrained(str(path), context_length=ctx)
     shape = getattr(synth, WL["shape"])
     ids = prompt_ids()
-    steps = max(1, min(args.steps, CTX - PROMPT - args.warmup - 1))
-    W = max(args.warmup, 3)
 
     def prefill():
         llm._context = []
@@ -413,6 +442,8 @@ def main():
     assert ms > 0
     ms = max_over_ranks(ms)
     tokens_dev = list(out[:steps])
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, llm, tokens_dev)                              # before the profiling passes below overwrite them
     replicas_agree = all(t == tokens_dev for t in group.gather_ints(tokens_dev))   # every replica decodes the same sequence
     value = replicas.aggregate_tokens_per_s(world, steps, ms)
 
@@ -453,7 +484,7 @@ def main():
     result = {
         "metric": METRIC, "value": value, "unit": "tokens/s", "n_gpus": world, "steps": steps, "warmup": W,
         "ms_per_step": ms / steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
-        "dtype": DTYPE, "data": "synthetic", "config": workload_config(world),
+        "dtype": DTYPE, "data": "synthetic", "config": workload_config(world, ctx),
         "clocks": clocks,
         "e2e": {"value": e2e, "unit": "tokens/s", "h2d_bytes_per_step": 16, "d2h_bytes_per_step": 8,
                 "how": "llm.eval([tok]) + llm.sample(top_k=1, repetition_penalty=1.0) per step, wall clock between device syncs; per step: H2D {token, position, step, n_total} (16 B), D2H {arg-max of the logits, number of logits equal to it} (8 B) — a greedy sample() is answered by the pick the engine made on the device (a sampled one would add the 64-token window up and a 2 KB candidate block down); the logits stay on the device until llm.logits is asked for",

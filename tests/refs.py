@@ -1,13 +1,16 @@
 """ctypes loaders for the two CHECKERS (test infrastructure, never the product):
 
   * ``oracle()``  — oracle/_build/liboracle.so, our plain-C restatement (oracle/ggml_oracle.c)
-  * ``ref()``     — oracle/_ref/libctransformers_ref.so, the unmodified reference compiled from
-                    /root/reference by oracle/Makefile (present when it was built in the container;
-                    it travels to the GPU box with the snapshot)
+  * ``ref()``     — oracle/_ref/libctransformers_ref.so, the unmodified reference compiled from its
+                    sources by oracle/Makefile (only where those sources are present); the tests
+                    compare with what it produced through tests/golden/, tests/golden/make_golden.py
+                    regenerates that data from it
 """
 import ctypes as C
+import hashlib
 import os
 import subprocess
+import zlib
 from pathlib import Path
 
 import numpy as np
@@ -15,6 +18,7 @@ import numpy as np
 ROOT = Path(__file__).resolve().parent.parent
 ORACLE_SO = ROOT / "oracle" / "_build" / "liboracle.so"
 REF_SO = ROOT / "oracle" / "_ref" / "libctransformers_ref.so"
+GOLD = ROOT / "tests" / "golden"
 
 # ggml type ids (ggml.h enum ggml_type)
 F32, F16, Q4_0, Q5_0, Q8_0, Q4_K, Q5_K, Q6_K, Q8_K = 0, 1, 2, 6, 8, 12, 13, 14, 15
@@ -124,6 +128,45 @@ def ref_vec_dot(t, k, wrow, act):
     s = np.zeros(1, dtype=np.float32)
     ref_traits(t)["vec_dot"](k, ptr(s), ptr(wrow), ptr(act))
     return float(s[0])
+
+
+# --------------------------------------------------------------------------------------------------------------
+# Stored reference results (tests/golden/make_golden.py writes them from the compiled reference)
+def digest(a):
+    """SHA-256 of an array's bytes: equal digests <=> bit-identical results (float32 for float arrays)."""
+    a = np.ascontiguousarray(a, np.float32 if np.asarray(a).dtype.kind == "f" else None)
+    return hashlib.sha256(a.tobytes()).hexdigest()
+
+
+def run_digests(run):
+    """modelcases.run_greedy's result as stored: digests of the first logits, first embeddings, last logits."""
+    return [digest(run[0]), digest(run[1]), digest(run[3])]
+
+
+_golden = {}
+
+
+def golden(name):
+    if name not in _golden:
+        _golden[name] = dict(np.load(GOLD / f"{name}.npz"))
+    return _golden[name]
+
+
+def pool_matrix(t, m, k, rng):
+    """[m, k] weights of type t made of blocks the reference's quantizer produced (tests/golden/ref_quant_pool.npz, from
+    seeded N(0.01, 0.05²) rows): every scale / min bit pattern the real quantizer emits, drawn block by block with rng."""
+    pool = golden("ref_quant_pool")[f"pool_{t}"]
+    bs, _ = BLOCK[t]
+    assert k % bs == 0
+    return np.ascontiguousarray(pool[rng.integers(0, len(pool), m * (k // bs))]).reshape(-1)
+
+
+def pool_quantizer(t, w):
+    """synth.write_* quantizer that stands in for the reference's: blocks from the stored pool, drawn with a rng seeded
+    from the f32 tensor the writer passes (so each tensor gets its own, reproducible draw)."""
+    w = np.ascontiguousarray(w, np.float32)
+    rng = np.random.default_rng(zlib.crc32(w[:4].tobytes()))
+    return pool_matrix(t, w.shape[0], w.shape[1], rng)
 
 
 # --------------------------------------------------------------------------------------------------------------

@@ -10,7 +10,6 @@ import pytest
 import refs
 from ctransformers_b200 import AutoModelForCausalLM, synth
 
-pytestmark = pytest.mark.skipif(not refs.have_ref(), reason="oracle/_ref (the compiled reference) is not present")
 
 
 @pytest.fixture(scope="module")
@@ -32,6 +31,7 @@ def run(path, n_new=32):
     return llm, first, toks
 
 
+@pytest.mark.skipif(not refs.have_ref(), reason="needs oracle/_ref, the reference compiled from its sources (make -C oracle ref)")
 def test_reference_runs_the_gpt2_file_through_this_python_surface(gpt2_file):
     path, shape = gpt2_file
     llm, first, toks = run(path)

@@ -1,6 +1,7 @@
 """GPU parity tests, whole path: synthetic GGUF models through the public Python API / the 17-function C ABI on the
-B200 library, against (1) the committed golden fixtures the reference produced (tests/golden/model_*.npz) and (2) the
-unmodified reference itself run live on the same file when oracle/_ref is present.
+B200 library, against (1) the committed golden fixtures the reference produced (tests/golden/model_*.npz) and (2) what
+the unmodified reference produced on the same files for further chunkings, prompts and models (tests/golden/reference_runs.npz:
+digests of its logits and hidden states, which must match bit for bit, and its greedy tokens).
 
 Bar: the north star asks for logits within 1e-3 relative and identical greedy tokens; the kernels reproduce the
 reference's accumulation order, so these tests demand the stronger thing — logits, embeddings and tokens IDENTICAL to the
@@ -21,6 +22,13 @@ LOGIT_TOL = 1e-3
 
 def rel_err(a, b):
     return float(np.abs(a - b).max() / np.abs(b).max())
+
+
+def same_as_reference(ours, key):
+    """A modelcases.run_greedy result against the reference's stored one: same tokens, bit-identical logits and hidden state."""
+    gold = refs.golden("reference_runs")
+    assert ours[2] == gold[key + "_tokens"].tolist()
+    assert refs.run_digests(ours) == gold[key + "_digests"].tolist(), "first logits / first embeddings / last logits differ from the reference's"
 
 
 def same_bits(a, b):
@@ -52,32 +60,22 @@ def test_against_golden_fixture(name, model_dir):
     same_bits(last_logits, gold["last_logits"])
 
 
-@pytest.mark.skipif(not refs.have_ref(), reason="oracle/_ref not present")
 @pytest.mark.parametrize("name", ["llama_tiny_q4km", "llama_gqa_q5km", "falcon_tiny_q5km"])
 def test_against_live_reference(name, model_dir):
     path, ctx = modelcases.build(name, model_dir)
     prompt = modelcases.prompt_for(name)
     for bs in (8, 64, 5):   # the chunking is part of the contract: it fixes the row length of the attention mat-muls
-        ours = modelcases.run_greedy(load(path, ctx), prompt, modelcases.N_NEW, batch_size=bs)
-        theirs = modelcases.run_greedy(load(path, ctx, lib=str(refs.REF_SO), threads=4), prompt, modelcases.N_NEW, batch_size=bs)
-        same_bits(ours[0], theirs[0])
-        same_bits(ours[1], theirs[1])
-        assert ours[2] == theirs[2]
-        same_bits(ours[3], theirs[3])
+        same_as_reference(modelcases.run_greedy(load(path, ctx), prompt, modelcases.N_NEW, batch_size=bs), f"live_{name}_{bs}")
 
 
-@pytest.mark.skipif(not refs.have_ref(), reason="oracle/_ref not present")
 def test_real_quantized_weights_against_live_reference(model_dir):
-    """Weights quantized by the reference's own quantizer from seeded f32 (not random blocks)."""
+    """Weights made by the reference's own quantizer (blocks of tests/golden/ref_quant_pool.npz), not random blocks."""
     from ctransformers_b200 import synth
     path = model_dir / "realq.gguf"
     shape = synth.LlamaShape(n_vocab=1024, n_embd=512, n_head=4, n_head_kv=4, n_ff=1536, n_layer=2, n_ctx_train=128)
-    synth.write_llama(path, shape, "Q4_K_M", seed=3, quantizer=lambda t, w: refs.ref_quantize(t, w), sigma=0.05)
+    synth.write_llama(path, shape, "Q4_K_M", seed=3, quantizer=refs.pool_quantizer, sigma=0.05)
     prompt = [1] + np.random.default_rng(0).integers(259, 1024, 30).tolist()
-    ours = modelcases.run_greedy(load(path, 64), prompt, 8)
-    theirs = modelcases.run_greedy(load(path, 64, lib=str(refs.REF_SO), threads=4), prompt, 8)
-    same_bits(ours[0], theirs[0])
-    assert ours[2] == theirs[2]
+    same_as_reference(modelcases.run_greedy(load(path, 64), prompt, 8), "realq")
 
 
 def test_logits_are_a_mutable_view_and_sampling_sees_edits(model_dir):
@@ -180,30 +178,21 @@ def test_greedy_lookahead_hits_and_misses_match_the_oracle(model_dir, lib):
     assert llm.ctb_llm_speculative_hits() - hits0 >= 4
 
 
-# ---- BASELINE-size models (configs[1] and configs[3]) against the live reference: the same files bench.py times
-@pytest.mark.skipif(not refs.have_ref(), reason="oracle/_ref not present")
+# ---- BASELINE-size models (configs[1] and configs[3]) against the reference: the same files bench.py times
 @pytest.mark.parametrize("workload", ["llama2-7b", "falcon7b"])
 def test_bench_model_against_live_reference(workload):
     """32-token prompt (reference default chunking, batch_size 8) + 8 greedy steps on the 7B-shaped bench model: logits after
     the prompt, the greedy tokens and the last logits must be the reference's, bit for bit."""
-    import os
     import sys
     sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
     import bench
     bench.WL = bench.WORKLOADS[workload]
-    path = bench.ensure_model(0, 1, lambda: None)          # /tmp/ctb_models (shared with bench.py on the same box)
+    path = bench.ensure_model(0, 1, lambda: None)          # bench.MODEL_DIR, shared with bench.py on the same machine
     prompt = bench.prompt_ids()[:32]
-    cores = os.cpu_count() or 1
-    ours = modelcases.run_greedy(load(path, 128), prompt, 8)
-    theirs = modelcases.run_greedy(load(path, 128, lib=str(refs.REF_SO), threads=min(16, cores)), prompt, 8)
-    same_bits(ours[0], theirs[0])
-    same_bits(ours[1], theirs[1])
-    assert ours[2] == theirs[2]
-    same_bits(ours[3], theirs[3])
+    same_as_reference(modelcases.run_greedy(load(path, 128), prompt, 8), f"bench_{workload}")
 
 
 # ---- batched prefill (csrc/prefill.cuh): prompts longer than a few tokens go through the dense int8 tensor-core kernel
-@pytest.mark.skipif(not refs.have_ref(), reason="oracle/_ref not present")
 @pytest.mark.parametrize("name,bs", [("llama_wide_q4km", 512), ("llama_wide_q4km", 64), ("llama_gqa_q5km", 5), ("falcon_tiny_q5km", 512)])
 def test_prefill_against_live_reference(name, bs, model_dir):
     """A prompt of 70 tokens (3 batched launches: 32 + 32 + 6) at batch_size 5 / 64 / 512: logits and hidden state after the
@@ -214,12 +203,7 @@ def test_prefill_against_live_reference(name, bs, model_dir):
     prompt = rng.integers(259 if arch == "llama" else 0, shape.n_vocab, 70).tolist()
     if arch == "llama":
         prompt[0] = 1
-    ours = modelcases.run_greedy(load(path, 96), prompt, 6, batch_size=bs)
-    theirs = modelcases.run_greedy(load(path, 96, lib=str(refs.REF_SO), threads=4), prompt, 6, batch_size=bs)
-    same_bits(ours[0], theirs[0])
-    same_bits(ours[1], theirs[1])
-    assert ours[2] == theirs[2]
-    same_bits(ours[3], theirs[3])
+    same_as_reference(modelcases.run_greedy(load(path, 96), prompt, 6, batch_size=bs), f"prefill_{name}_{bs}")
 
 
 def test_prefill_equals_single_token_path(model_dir, monkeypatch):

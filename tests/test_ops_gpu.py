@@ -217,15 +217,15 @@ def test_get_row_bit_exact(lib, t):
         assert np.array_equal(got.view(np.uint32), np.ascontiguousarray(want[r]).view(np.uint32))
 
 
-@pytest.mark.skipif(not refs.have_ref(), reason="oracle/_ref not present")
 @pytest.mark.parametrize("t", [Q4_K, Q5_K, Q6_K, Q4_0, Q5_0, Q8_0])
 @pytest.mark.parametrize("k", [512, 1024, 2816])
 def test_mul_mat_real_quantized_weights(lib, t, k):
-    """Weights produced by the reference's quantizer (all scale/min bit patterns occur, unlike the random-block generator)."""
+    """Weights made of blocks the reference's quantizer produced (all scale/min bit patterns occur, unlike the random-block
+    generator): tests/golden/ref_quant_pool.npz."""
     o = refs.oracle()
     rng = np.random.default_rng(k + t)
     m = 48
-    w = refs.ref_quantize(t, (rng.standard_normal((m, k)) * 0.05 + 0.01).astype(np.float32))
+    w = refs.pool_matrix(t, m, k, rng)
     x = _act(rng, k)[None]
     want, got = np.zeros((1, m), np.float32), np.zeros((1, m), np.float32)
     assert o.orc_mul_mat(t, ptr(w), ptr(x), ptr(want), k, m, 1) == 0

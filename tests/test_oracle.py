@@ -1,6 +1,6 @@
 """CPU tests that pin the oracle: the plain-C restatement (oracle/ggml_oracle.c) against (1) the committed golden
-vectors that the unmodified reference produced (tests/golden/make_golden.py), (2) the compiled reference itself when
-oracle/_ref is present, (3) the known-answer thresholds of upstream test-quantize-fns.cpp
+vectors that the unmodified reference produced (tests/golden/make_golden.py), (2) what the compiled reference produced
+for the inputs the tests below build (tests/golden/reference_runs.npz), (3) the known-answer thresholds of upstream test-quantize-fns.cpp
 (models/submodules/llama.cpp/tests/test-quantize-fns.cpp:16-31, 76-113)."""
 from pathlib import Path
 
@@ -82,38 +82,45 @@ def test_fp16_conversions_exhaustive():
     assert np.array_equal(np.array([o.orc_fp32_to_fp16(float(v)) for v in x], np.uint16), x.astype(np.float16).view(np.uint16))
 
 
-@pytest.mark.skipif(not refs.have_ref(), reason="oracle/_ref not built (needs /root/reference)")
 class TestAgainstCompiledReference:
+    """Against what the compiled reference produced for the same seeded inputs (tests/golden/reference_runs.npz)."""
+
     def test_quantizers_bit_exact(self):
+        gold = refs.golden("reference_runs")
         rng = np.random.default_rng(7)
         for trial in range(60):
             x = (rng.standard_normal(2048) * rng.choice([1e-3, 1, 50])).astype(np.float32)
             if trial % 7 == 0:
                 x[256:512] = 0
-            for t in (Q8_K, Q8_0):
-                assert np.array_equal(refs.ref_quantize_act(t, x), _oracle_quant(t, x))
+            assert refs.digest(_oracle_quant(Q8_K, x)) == gold["quant_q8k"][trial], trial
+            assert refs.digest(_oracle_quant(Q8_0, x)) == gold["quant_q80"][trial], trial
 
     @pytest.mark.parametrize("t,at", TYPES)
     def test_vec_dot(self, t, at):
+        """Weights from the reference's quantizer, activations quantized by the oracle (identical to the reference's)."""
+        gold = refs.golden("reference_runs")
         o = refs.oracle()
         rng = np.random.default_rng(t)
         k = 4096
-        w = (rng.standard_normal((16, k)) * 0.02).astype(np.float32)
+        wq = refs.pool_matrix(t, 16, k, rng).reshape(16, -1)
         x = rng.standard_normal(k).astype(np.float32)
-        wq = refs.ref_quantize(t, w).reshape(16, -1)
-        act = refs.ref_quantize_act(at, x)
+        act = _oracle_quant(at, x)
+        assert refs.digest(act) == gold[f"vecdot_act_{t}"]
         fn = getattr(o, f"orc_vec_dot_{refs.TYPE_NAME[t]}_{'q8_K' if at == Q8_K else 'q8_0'}")
-        for i in range(16):
-            a, b = np.float32(refs.ref_vec_dot(t, k, wq[i], act)), np.float32(fn(k, ptr(wq[i]), ptr(act)))
-            assert a.view(np.uint32) == b.view(np.uint32)
+        got = np.array([fn(k, ptr(np.ascontiguousarray(wq[i])), ptr(act)) for i in range(16)], np.float32)
+        assert np.array_equal(got.view(np.uint32), gold[f"vecdot_{t}"].view(np.uint32))
 
     def test_random_block_generator_is_valid_for_the_reference(self):
-        """synth.random_blocks must produce blocks the reference dequantizes to finite, sensibly scaled weights."""
+        """synth.random_blocks must produce blocks the reference dequantizes to finite, sensibly scaled weights (the oracle's
+        dequantization of them is checked to be the reference's, bit for bit)."""
         from ctransformers_b200 import synth
+        gold = refs.golden("reference_runs")
+        o = refs.oracle()
         for t in (Q4_0, Q5_0, Q8_0, Q4_K, Q5_K, Q6_K):
             blocks = np.ascontiguousarray(synth.random_blocks(t, 1024, 8, 0.02, np.random.default_rng(t)))
             out = np.zeros(8 * 1024, np.float32)
-            refs.ref_traits(t)["to_float"](ptr(blocks), ptr(out), out.size)
+            getattr(o, "orc_dequantize_row_" + refs.TYPE_NAME[t])(ptr(blocks), ptr(out), out.size)
+            assert refs.digest(out) == gold[f"randblk_deq_{t}"], t
             assert np.isfinite(out).all()
             assert 0.01 < out.std() < 0.04, (t, out.std())
             assert abs(out.mean()) < 0.004
@@ -140,22 +147,17 @@ def test_full_eval_matches_reference_golden(name, tmp_path_factory):
     assert toks == gold["tokens"][:6].tolist()
 
 
-@pytest.mark.skipif(not refs.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("name", ["llama_tiny_q4km", "falcon_tiny_q5km"])
 def test_full_eval_matches_live_reference_for_any_chunking(name, tmp_path_factory):
-    """70-token prompt (so the V·P f16 dot uses both its SIMD part and its scalar tail), three chunkings, then 3 decode steps."""
-    from ctransformers_b200 import AutoModelForCausalLM
+    """70-token prompt (so the V·P f16 dot uses both its SIMD part and its scalar tail), three chunkings, then 3 decode steps:
+    every logits vector is the reference's for the same chunking (tests/golden/reference_runs.npz)."""
+    gold = refs.golden("reference_runs")
     path, ctx = modelcases.build(name, tmp_path_factory.mktemp("orc_live"))
     arch, shape, _, _ = modelcases.CASES[name]
     ids = np.random.default_rng(9).integers(259 if arch == "llama" else 0, shape.n_vocab, 70).tolist()
     for bs in (8, 64, 33):
-        ref = AutoModelForCausalLM.from_pretrained(str(path), lib=str(refs.REF_SO), context_length=ctx, threads=4)
-        ref.eval(ids, batch_size=bs)
         m = refs.OracleModel(path, ctx)
         m.eval(ids, batch_size=bs)
-        for _ in range(3):
-            a = np.array(ref.logits, dtype=np.float32)
-            assert np.array_equal(a.view(np.uint32), m.logits.view(np.uint32))
-            t = int(np.argmax(a))
-            ref.eval([t])
-            m.eval([t])
+        for step in range(3):
+            assert refs.digest(m.logits) == gold[f"chunk_{name}_{bs}"][step], (bs, step)
+            m.eval([int(np.argmax(m.logits))])
